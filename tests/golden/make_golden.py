@@ -1,7 +1,9 @@
 #!/usr/bin/env python3
 """Generates tests/golden/kats.json from the reference's own Rust test sources.
 
-Run HERE (the container that has /root/reference); the GPU box never sees the reference.
+    python tests/golden/make_golden.py <checkout of LayerXcom/zero-chain>
+
+The tests only read what this script writes under tests/golden/; they never need the reference itself.
 Only numeric literals (known-answer vectors) are extracted — no reference code is copied.
 For each listed `#[test] fn`, the ordered list of `FqRepr([..])` / `FrRepr([..])` limb groups
 (little-endian u64 limbs as written in the source) is recorded; tests/test_oracle_kats.py
@@ -12,9 +14,6 @@ encoding vector files and the shipped CRS files) so the oracle-generated equival
 compared without committing the reference's files.
 """
 import hashlib, json, os, re, sys
-
-REF = os.environ.get("ZK_REFERENCE", "/root/reference")
-BLS = os.path.join(REF, "core/pairing/src/bls12_381")
 
 TESTS = {
     "fq.rs": ["test_fq_add_assign", "test_fq_sub_assign", "test_fq_mul_assign", "test_fq_squaring",
@@ -40,6 +39,9 @@ FILES = [
     "zface/params/anony_pk.dat",
     "core/bellman-verifier/src/tests/proving.params",
 ]
+# points kept from each query of the shipped conf_pk.dat: about 1/32 of it, so the fixture stays small (the whole file is
+# 10 MB).  The counts form a consistent proving key of a smaller circuit: h = 2^10 - 1, l = n_aux, a = 23 inputs + 486 aux.
+SAMPLE_COUNTS = {"h": 1023, "l": 623, "a": 509, "b_g1": 387, "b_g2": 387}
 GROUP = re.compile(r"F[qr]Repr\(\[\s*((?:0x[0-9a-fA-F_]+\s*,?\s*)+)\]\)")
 
 
@@ -62,7 +64,23 @@ def groups(text):
     return out
 
 
+def params_sample(pk):
+    """The vk of `pk` unchanged (alpha .. delta, all ic points), then the first SAMPLE_COUNTS[q] points of every query q, in
+    Parameters::write's grammar."""
+    vk_len = 868 + 96 * int.from_bytes(pk[864:868], "big")
+    out, off, full = bytearray(pk[:vk_len]), vk_len, {}
+    for q, sz in (("h", 96), ("l", 96), ("a", 96), ("b_g1", 96), ("b_g2", 192)):
+        n = int.from_bytes(pk[off:off + 4], "big")
+        full[q] = n
+        out += SAMPLE_COUNTS[q].to_bytes(4, "big") + pk[off + 4:off + 4 + sz * SAMPLE_COUNTS[q]]
+        off += 4 + sz * n
+    assert off == len(pk)
+    return bytes(out), full
+
+
 def main():
+    REF = sys.argv[1]
+    BLS = os.path.join(REF, "core/pairing/src/bls12_381")
     res = {"source": "LayerXcom/zero-chain core/pairing/src/bls12_381", "tests": {}, "consts": {}, "files": {}}
     for f, names in TESTS.items():
         src = open(os.path.join(BLS, f)).read()
@@ -100,10 +118,14 @@ def main():
         n_ic = int.from_bytes(pkb[864:868], "big")
         open(os.path.join(here, "%s_vk_head.bin" % name), "wb").write(pkb[:868 + 96 * n_ic])
         open(os.path.join(here, "%s_pvk.dat" % name), "wb").write(open(os.path.join(REF, "zface/params/%s_vk.dat" % name), "rb").read())
-    # the shipped confidential-transfer CRS itself (10 133 592 B, 93 124 points): the GPU box has no /root/reference, and
-    # Parameters::read(&pk_buf[..], true) on exactly these bytes (core/proofs/src/confidential.rs:95-103) is what the
-    # device loader replaces — tests/test_gpu_real_crs.py loads it, proves on it and round-trips it through zk_params_write
-    open(os.path.join(here, "conf_pk.dat"), "wb").write(open(os.path.join(REF, "zface/params/conf_pk.dat"), "rb").read())
+    # a sample of the shipped confidential-transfer CRS (10 133 592 B, 93 124 points): Parameters::read(&pk_buf[..], true)
+    # (core/proofs/src/confidential.rs:95-103) is what the device loader replaces, and these points were not made by this
+    # repository's code — tests/test_gpu_real_crs.py loads the sample, proves on it and round-trips it through zk_params_write
+    sample, full = params_sample(open(os.path.join(REF, "zface/params/conf_pk.dat"), "rb").read())
+    open(os.path.join(here, "conf_pk_sample.dat"), "wb").write(sample)
+    res["conf_pk_sample"] = {"source": "zface/params/conf_pk.dat: its vk, then the first points of every query",
+                             "full_counts": full, "counts": SAMPLE_COUNTS,
+                             "size": len(sample), "sha256": hashlib.sha256(sample).hexdigest()}
     out = os.path.join(os.path.dirname(os.path.abspath(__file__)), "kats.json")
     json.dump(res, open(out, "w"), indent=1)
     print("wrote", out, {k: len(v["groups"]) for k, v in res["tests"].items()})

@@ -1,11 +1,12 @@
-"""GPU parity tests on the reference's SHIPPED proving key (zface/params/conf_pk.dat, committed as tests/golden/conf_pk.dat by
-tests/golden/make_golden.py): the call the device loader replaces is `Parameters::read(&pk_buf[..], true)` at
-core/proofs/src/confidential.rs:95-103, the writer `self.proving_key.write(..)` at confidential.rs:73-93.
+"""GPU parity tests on a sample of the reference's SHIPPED proving key (zface/params/conf_pk.dat: its vk and the first points of
+every query, committed as tests/golden/conf_pk_sample.dat by tests/golden/make_golden.py): the call the device loader replaces
+is `Parameters::read(&pk_buf[..], true)` at core/proofs/src/confidential.rs:95-103, the writer `self.proving_key.write(..)` at
+confidential.rs:73-93.
 
-Every toy CRS in the other tests consists of known multiples of the generator made by this repo's own code; the 93 124 points of
-this file are not, so a decoding or group-law defect that only "foreign" points trigger shows up here.  A real
+Every toy CRS in the other tests consists of known multiples of the generator made by this repo's own code; the 2 952 points of
+the sample are not, so a decoding or group-law defect that only "foreign" points trigger shows up here.  A real
 confidential_transfer witness cannot be made here (it needs the Rust gadget library), so the proofs use a synthetic assignment of
-the real shape — they do not verify under conf_vk.dat, but their bytes must equal the oracle's on the same CRS and inputs."""
+the sample's shape — they do not verify under conf_vk.dat, but their bytes must equal the oracle's on the same CRS and inputs."""
 import hashlib
 import json
 import os
@@ -20,7 +21,9 @@ from zero_chain_b200 import synthetic as sy
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-COUNTS = (23, 32767, 19955, 15598, 12402, 12402)          # ic, h, l, a, b_g1, b_g2 (SURVEY.md §8 a10)
+COUNTS = (23, 1023, 623, 509, 387, 387)                   # ic, h, l, a, b_g1, b_g2 of the sample (about 1/32 of every query)
+# the circuit the sample is the proving key of: domain 2^10, a = inputs + a_aux_density, b = b_density
+SHAPE = dict(n_constraints=624, n_inputs=23, n_aux=623, a_aux_density=486, b_density=387)
 
 
 @pytest.fixture(scope="module")
@@ -32,23 +35,23 @@ def ctx():
 
 @pytest.fixture(scope="module")
 def pk():
-    buf = open(os.path.join(GOLD, "conf_pk.dat"), "rb").read()
-    K = json.load(open(os.path.join(GOLD, "kats.json")))
-    assert len(buf) == 10133592 and hashlib.sha256(buf).hexdigest() == K["files"]["zface/params/conf_pk.dat"]["sha256"]
+    buf = open(os.path.join(GOLD, "conf_pk_sample.dat"), "rb").read()
+    S = json.load(open(os.path.join(GOLD, "kats.json")))["conf_pk_sample"]
+    assert len(buf) == S["size"] and hashlib.sha256(buf).hexdigest() == S["sha256"]
     return buf
 
 
 @pytest.fixture(scope="module")
 def params(ctx, pk):
-    p = zk.Parameters.read(ctx, pk, checked=True)          # on-curve + r-torsion tests of all 93 124 points on the device
+    p = zk.Parameters.read(ctx, pk, checked=True)          # on-curve + r-torsion tests of every point on the device
     yield p
     p.free()
 
 
 def _assignment(seed):
-    """A synthetic ProvingAssignment of the real circuit's shape: c = a * b on every row (so that H is a polynomial),
-    ~90 % of the aux values in {0, 1} like a boolean-heavy witness, densities with the real counts."""
-    sh = sy.CONF_SHAPE
+    """A synthetic ProvingAssignment of the sample's shape: c = a * b on every row (so that H is a polynomial),
+    ~90 % of the aux values in {0, 1} like a boolean-heavy witness, densities with the sample's counts."""
+    sh = SHAPE
     n_in, n_aux = sh["n_inputs"], sh["n_aux"]
     n_c = sh["n_constraints"] + n_in
     rng = sy.SplitMix64(seed)
@@ -70,7 +73,7 @@ def _oracle_prove(op, pa, r, s):
 
 def test_shipped_crs_loads_checked_and_round_trips(ctx, pk, params):
     assert (params.n_ic, params.n_h, params.n_l, params.n_a, params.n_b_g1, params.n_b_g2) == COUNTS
-    # Parameters::write of the resident CRS reproduces the shipped file byte for byte (decode -> Montgomery -> encode)
+    # Parameters::write of the resident CRS reproduces the sample byte for byte (decode -> Montgomery -> encode)
     out = params.write()
     assert len(out) == len(pk) and hashlib.sha256(out).digest() == hashlib.sha256(pk).digest() and out == pk
     # params.vk (setup.rs:31) and prepare_verifying_key of it = the shipped conf_vk.dat
@@ -105,7 +108,7 @@ def test_proofs_on_the_shipped_crs_equal_the_oracle(ctx, pk, params):
 
 def test_corrupted_shipped_crs_is_rejected(ctx, pk):
     lay = pr.params_layout(pk)
-    off = lay["a"][0] + 96 * 777
+    off = lay["a"][0] + 96 * (lay["a"][1] * 3 // 4)
     bad = bytearray(pk); bad[off + 95] ^= 1                                   # y changed: not on the curve
     with pytest.raises(zk.SynthesisError) as e:
         zk.Parameters.read(ctx, bytes(bad), checked=True)
@@ -118,7 +121,7 @@ def test_corrupted_shipped_crs_is_rejected(ctx, pk):
         if y is not None and pr.ec_mul(pr.FQ, (x, y), pr.R) is not pr.INF:
             break
         x += 1
-    off = lay["h"][0] + 96 * 31000
+    off = lay["h"][0] + 96 * (lay["h"][1] - 30)
     bad = bytearray(pk); bad[off:off + 96] = x.to_bytes(48, "big") + y.to_bytes(48, "big")
     with pytest.raises(zk.SynthesisError) as e:
         zk.Parameters.read(ctx, bytes(bad), checked=True)
@@ -138,7 +141,7 @@ def test_decoded_crs_cache(ctx, pk, params, tmp_path):
     pa = _assignment(7)
     want = zk.create_proof(pa, params, 11, 22)
     p1 = zk.Parameters.read_cached(ctx, pk, path)
-    assert not p1.cache_hit and os.path.getsize(path) > 9_000_000
+    assert not p1.cache_hit and os.path.getsize(path) > 0.9 * len(pk)
     p2 = zk.Parameters.read_cached(ctx, pk, path)
     assert p2.cache_hit
     for p in (p1, p2):
@@ -150,13 +153,13 @@ def test_decoded_crs_cache(ctx, pk, params, tmp_path):
         zk.Parameters.read_cached(ctx, bytes(other), path)
     # a cache whose BODY was altered (header intact) must not be trusted: it is ignored and rewritten
     with open(path, "r+b") as f:
-        f.seek(5_000_000); b = f.read(1); f.seek(5_000_000); f.write(bytes([b[0] ^ 1]))
+        f.seek(len(pk) // 2); b = f.read(1); f.seek(len(pk) // 2); f.write(bytes([b[0] ^ 1]))
     p4 = zk.Parameters.read_cached(ctx, pk, path)
     assert not p4.cache_hit and zk.create_proof(pa, p4, 11, 22) == want
     p4.free()
     assert zk.Parameters.read_cached(ctx, pk, path).cache_hit
     # a truncated cache file is ignored and rewritten
-    open(path, "r+b").truncate(1 << 20)
+    open(path, "r+b").truncate(len(pk) // 10)
     p3 = zk.Parameters.read_cached(ctx, pk, path)
-    assert not p3.cache_hit and os.path.getsize(path) > 9_000_000
+    assert not p3.cache_hit and os.path.getsize(path) > 0.9 * len(pk)
     p3.free()

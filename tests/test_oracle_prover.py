@@ -160,19 +160,21 @@ def test_params_read_errors():
 
 
 def test_shipped_crs_parses():
-    """Parameters grammar vs the reference's shipped CRS (tests/golden/conf_pk.dat, copied from zface/params/conf_pk.dat by
-    tests/golden/make_golden.py, so the GPU box sees the same bytes).  SURVEY.md §3.3: the grammar must consume all bytes."""
+    """Parameters grammar vs a sample of the reference's shipped CRS (tests/golden/conf_pk_sample.dat: the vk of
+    zface/params/conf_pk.dat and the first points of every query, written by tests/golden/make_golden.py with the query
+    lengths of the whole file).  SURVEY.md §3.3: the grammar must consume all bytes."""
     import hashlib, json, os
-    path = os.path.join(os.path.dirname(__file__), "golden", "conf_pk.dat")
-    buf = open(path, "rb").read()
-    ref = "/root/reference/zface/params/conf_pk.dat"
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == buf
-    K = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "kats.json")))
-    assert hashlib.sha256(buf).hexdigest() == K["files"]["zface/params/conf_pk.dat"]["sha256"]
+    gold = os.path.join(os.path.dirname(__file__), "golden")
+    buf = open(os.path.join(gold, "conf_pk_sample.dat"), "rb").read()
+    S = json.load(open(os.path.join(gold, "kats.json")))["conf_pk_sample"]
+    assert hashlib.sha256(buf).hexdigest() == S["sha256"]
+    assert buf.startswith(open(os.path.join(gold, "conf_vk_head.bin"), "rb").read())
     lay = pr.params_layout(buf)
-    assert lay["end"][0] == len(buf) == 10133592
-    P = co.Params(buf, checked=True)          # on-curve + r-torsion for all 93 124 points
-    assert (P.n_ic, P.n_h, P.n_l, P.n_a, P.n_b) == (23, 32767, 19955, 15598, 12402)
+    assert lay["end"][0] == len(buf) == S["size"]
+    P = co.Params(buf, checked=True)          # on-curve + r-torsion for every point of the sample
+    assert (P.n_ic, P.n_h, P.n_l, P.n_a, P.n_b) == (23,) + tuple(S["counts"][q] for q in ("h", "l", "a", "b_g1"))
+    # the query lengths of the whole shipped file are the shape of the synthetic circuit
+    full = S["full_counts"]
+    assert (full["h"], full["l"], full["a"], full["b_g1"], full["b_g2"]) == (32767, 19955, 15598, 12402, 12402)
     sh = sy.CONF_SHAPE
-    assert P.n_h == (1 << 15) - 1 and P.n_l == sh["n_aux"] and P.n_a == sh["n_inputs"] + sh["a_aux_density"] and P.n_b == sh["b_density"]
+    assert full["h"] == (1 << 15) - 1 and full["l"] == sh["n_aux"] and full["a"] == sh["n_inputs"] + sh["a_aux_density"] and full["b_g1"] == sh["b_density"]
