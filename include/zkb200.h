@@ -44,6 +44,7 @@ extern "C" {
 #define ZK_ERR_DECODE (-7)               /* GroupDecodingError (not on curve, not in subgroup, bad flags, x >= q) */
 #define ZK_ERR_NOT_CANONICAL (-8)        /* a scalar >= r (PrimeFieldDecodingError::NotInField) */
 #define ZK_ERR_MALFORMED_VK (-9)         /* SynthesisError::MalformedVerifyingKey: inputs.len() + 1 != ic.len() */
+#define ZK_ERR_UNCONSTRAINED_VARIABLE (-10)  /* SynthesisError::UnconstrainedVariable: an L-query point is the identity */
 
 const char *zk_last_error(void);
 int zk_device_count(void);
@@ -188,9 +189,25 @@ int zk_groth16_prove_witness_batch(zk_ctx *ctx, const zk_params *p, const zk_r1c
                                    const uint64_t *input_assignment, const uint64_t *aux_assignment,
                                    const uint64_t *r, const uint64_t *s, uint8_t *proofs_out);
 
+/* ---- parameter generation (replaces bellman::groth16::generate_parameters) ---------------------------------------------
+ * generate_parameters (bellman groth16 generator.rs; reference calls core/proofs/src/setup.rs:28,59 through
+ * generate_random_parameters, which draws g1, g2, alpha, beta, gamma, delta, tau from the rng).
+ * r1cs: the circuit's constraints (zk_r1cs_load; the `input_i * 0 = 0` rows are appended here as in bellman).
+ * g1, g2: G1Uncompressed / G2Uncompressed, checked (on curve, r-torsion, not infinity).
+ * tau..delta: canonical FrRepr.  out: resident parameters, ready to prove with, equal to what zk_params_load would give
+ * for the bytes bellman's Parameters::write emits for the same inputs.
+ * Errors: ZK_ERR_NOT_CANONICAL (a scalar >= r), ZK_ERR_UNEXPECTED_IDENTITY (gamma or delta = 0 as in bellman; also alpha = 0,
+ * beta = 0, tau = 0 or tau^m = 1, whose points zk_params_load would reject; a generator at infinity), ZK_ERR_DECODE (a generator
+ * off the curve or outside the subgroup), ZK_ERR_UNCONSTRAINED_VARIABLE, ZK_ERR_POLY_DEGREE_TOO_LARGE (domain above 2^28 or a
+ * vector of 2^26 points or more), ZK_ERR_INVALID (r1cs on another device).  The device buffers that held the trapdoor or values
+ * derived from it are cleared before the call returns. */
+int zk_groth16_generate(zk_ctx *ctx, const zk_r1cs *r1cs, const uint8_t g1[96], const uint8_t g2[192],
+                        const uint64_t alpha[4], const uint64_t beta[4], const uint64_t gamma[4],
+                        const uint64_t delta[4], const uint64_t tau[4], zk_params **out);
+
 /* ---- utilities / diagnostics ------------------------------------------------------------------ */
-/* out[i] = scalars[i] * base (limb form in, limb form out); group 1 or 2.  Used to build synthetic
- * CRS / test vectors on the device (fixed-base scalar multiplication). */
+/* out[i] = scalars[i] * base (limb form in, limb form out); group 1 or 2; any 256-bit scalar.  Used to build synthetic
+ * CRS / test vectors on the device (the batched fixed-base multiplication of zk_groth16_generate). */
 int zk_scalar_mul_many(zk_ctx *ctx, int group, const uint64_t *base_limbs, const uint64_t *scalars, size_t n,
                        uint64_t *out_limbs);
 /* element-wise field ops on host arrays (parity tests of the device arithmetic):

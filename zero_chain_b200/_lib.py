@@ -53,6 +53,7 @@ SIGNATURES = {
     "zk_r1cs_load": (i32, [vp, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp, PP]),
     "zk_r1cs_free": (None, [vp]),
     "zk_groth16_prove_witness_batch": (i32, [vp, vp, vp, sz, vp, vp, vp, vp, vp]),
+    "zk_groth16_generate": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, PP]),
     "zk_scalar_mul_many": (i32, [vp, i32, vp, vp, sz, vp]),
     "zk_field_op": (i32, [vp, i32, i32, vp, vp, sz, vp]),
     "zk_bench_modmul": (i32, [vp, i32, i32, i32, i32, C.POINTER(dbl), C.POINTER(dbl)]),

@@ -53,7 +53,7 @@ extern "C" void zk_ctx_destroy(zk_ctx *c) {
                       &c->sorted, &c->partials, &c->buckets, &c->red_part, &c->red_x, &c->result, &c->out_bytes, &c->stage_a, &c->stage_b,
                       &c->stage_c, &c->ntt_tmp, &c->g_a, &c->g_b, &c->g_c, &c->g_h, &c->g_scal, &c->g_misc,
                       &c->aff_pts0, &c->aff_pts1, &c->aff_scratch, &c->aff_off0, &c->aff_off1, &c->aff_sizes0, &c->aff_sizes1, &c->aff_srcs, &c->aff_tot, &c->red_rows, &c->g_scal2, &c->g_scal3, &c->sorted2, &c->coarse_off, &c->coarse_sizes, &c->task_order, &c->len_hist, &c->heavy_list, &c->red_tmp,
-                      &c->v_pts, &c->v_stat, &c->v_coef, &c->v_f, &c->v_part, &c->v_io};
+                      &c->v_pts, &c->v_stat, &c->v_coef, &c->v_f, &c->v_part, &c->v_io, &c->fb_tbl};
     for (DevBuf *b : bufs) b->release();
     for (NttSlot &sl : c->ntt_slots) { sl.w.release(); sl.g.release(); sl.gi.release(); sl.consts.release(); }
     if (c->tail) { cudaStreamSynchronize(c->tail); cudaStreamDestroy(c->tail); cudaEventDestroy(c->ev_front); cudaEventDestroy(c->ev_tail); }
@@ -307,6 +307,9 @@ extern "C" int zk_points_fold(zk_ctx *ctx, int group, const void *d_partials, si
 }
 
 // ---- utilities -----------------------------------------------------------------------------------------------
+#ifdef ZK_EXPERIMENTS
+// the previous path, one thread per point with a full double-and-add; experiment builds select it with ZK_FB_OLD=1 so that
+// tools/setup_bench.py can compare the two on the same scalars
 template <class F>
 __global__ void __launch_bounds__(128) k_scalar_mul_many(const Affine<F> *base, const uint32_t *scalars, size_t n, Affine<F> *out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -315,6 +318,8 @@ __global__ void __launch_bounds__(128) k_scalar_mul_many(const Affine<F> *base, 
     for (int j = 0; j < 8; j++) k[j] = scalars[i * 8 + j];
     out[i] = scalar_mul(XYZZ<F>::from_affine(base[0]), k).to_affine();
 }
+#endif
+// the batched fixed-base multiplication of parameter generation (setup.cu): any 256-bit scalar, exact k * base
 extern "C" int zk_scalar_mul_many(zk_ctx *ctx, int group, const uint64_t *base, const uint64_t *scalars, size_t n, uint64_t *out) {
     if (!ctx || !base || !scalars || !out) { zk_set_error("zk_scalar_mul_many: NULL argument"); return ZK_ERR_INVALID; }
     if (group != 1 && group != 2) { zk_set_error("group must be 1 or 2"); return ZK_ERR_INVALID; }
@@ -323,10 +328,15 @@ extern "C" int zk_scalar_mul_many(zk_ctx *ctx, int group, const uint64_t *base, 
     ZK_TRY(ctx->stage_a.reserve(psz)); ZK_TRY(ctx->stage_b.reserve(n * 32)); ZK_TRY(ctx->stage_c.reserve(n * psz));
     ZK_CUDA(cudaMemcpyAsync(ctx->stage_a.p, base, psz, cudaMemcpyHostToDevice, ctx->stream));
     ZK_CUDA(cudaMemcpyAsync(ctx->stage_b.p, scalars, n * 32, cudaMemcpyHostToDevice, ctx->stream));
-    unsigned blk = (unsigned)((n + 127) / 128);
-    if (group == 1) k_scalar_mul_many<Fq><<<blk, 128, 0, ctx->stream>>>(ctx->stage_a.as<G1Affine>(), ctx->stage_b.as<uint32_t>(), n, ctx->stage_c.as<G1Affine>());
-    else k_scalar_mul_many<Fq2><<<blk, 128, 0, ctx->stream>>>(ctx->stage_a.as<G2Affine>(), ctx->stage_b.as<uint32_t>(), n, ctx->stage_c.as<G2Affine>());
-    ZK_CUDA(cudaGetLastError());
+#ifdef ZK_EXPERIMENTS
+    if (getenv("ZK_FB_OLD") && atoi(getenv("ZK_FB_OLD")) && n) {
+        unsigned blk = (unsigned)((n + 127) / 128);
+        if (group == 1) k_scalar_mul_many<Fq><<<blk, 128, 0, ctx->stream>>>(ctx->stage_a.as<G1Affine>(), ctx->stage_b.as<uint32_t>(), n, ctx->stage_c.as<G1Affine>());
+        else k_scalar_mul_many<Fq2><<<blk, 128, 0, ctx->stream>>>(ctx->stage_a.as<G2Affine>(), ctx->stage_b.as<uint32_t>(), n, ctx->stage_c.as<G2Affine>());
+        ZK_CUDA(cudaGetLastError());
+    } else
+#endif
+    ZK_TRY(zk_fixed_base(ctx, group, ctx->stage_a.p, ctx->stage_b.p, n, ctx->stage_c.p));
     ZK_CUDA(cudaMemcpyAsync(out, ctx->stage_c.p, n * psz, cudaMemcpyDeviceToHost, ctx->stream));
     ZK_CUDA(cudaStreamSynchronize(ctx->stream));
     return ZK_OK;

@@ -34,7 +34,7 @@ struct zk_params {
 // The fixed constraint system of one circuit, resident on the device in CSR form (SURVEY.md §8 f4).
 struct zk_r1cs {
     int device = 0;
-    size_t n_c = 0, n_in = 0, n_aux = 0;
+    size_t n_c = 0, n_in = 0, n_aux = 0, nnz[3] = {0, 0, 0};
     uint32_t *d_row_ptr[3] = {nullptr, nullptr, nullptr}, *d_col[3] = {nullptr, nullptr, nullptr};
     void *d_coeff[3] = {nullptr, nullptr, nullptr};
     std::vector<uint8_t> a_aux_density, b_input_density, b_aux_density;     // DensityTracker bits, derived from A and B
@@ -636,6 +636,7 @@ extern "C" int zk_r1cs_load(zk_ctx *ctx, size_t n_constraints, size_t n_inputs, 
     q->a_aux_density.assign(n_aux ? n_aux : 1, 0); q->b_input_density.assign(n_inputs, 0); q->b_aux_density.assign(n_aux ? n_aux : 1, 0);
     for (int w = 0; w < 3; w++) {
         size_t nnz = rp[w][n_constraints];
+        q->nnz[w] = nnz;
         if (rp[w][0] != 0 || (nnz && (!cl[w] || !cf[w]))) { zk_r1cs_free(q); zk_set_error("zk_r1cs_load: malformed CSR"); return ZK_ERR_INVALID; }
         for (size_t j = 0; j < n_constraints; j++) if (rp[w][j] > rp[w][j + 1]) { zk_r1cs_free(q); zk_set_error("zk_r1cs_load: row_ptr not monotone"); return ZK_ERR_INVALID; }
         for (size_t k = 0; k < nnz; k++) {
@@ -670,5 +671,122 @@ extern "C" int zk_groth16_prove_witness_batch(zk_ctx *ctx, const zk_params *p, c
         ZK_TRY(prove_impl(ctx, p, k, nullptr, nullptr, nullptr, 0, inputs + o * q->n_in * 4, q->n_in, aux + o * q->n_aux * 4, q->n_aux, nullptr, nullptr, nullptr,
                           r + o * 4, s + o * 4, proofs_out + o * 192, q));
     }
+    return ZK_OK;
+}
+
+// ---- generate_parameters (bellman groth16 generator.rs; reference calls core/proofs/src/setup.rs:28,59) ---------------------------
+// Same algebra as bellman, on the device: powers of tau -> IFFT = the Lagrange coefficients at tau; at / bt / ct per variable = the
+// coefficients summed over each matrix column (zk_setup_qap); the query scalars in CrsLayout order; one fixed-base launch for all G1
+// scalars and one for all G2 scalars (zk_fixed_base); then the window tables as for a loaded CRS.  Every group element is unique and
+// so is its uncompressed encoding: zk_params_write of the result equals what Parameters::write emits for the same inputs.
+namespace {
+const uint64_t FR_R[4] = {0xffffffff00000001ull, 0x53bda402fffe5bfeull, 0x3339d80809a1d805ull, 0x73eda753299d7d48ull};
+bool fr_canonical(const uint64_t *k) {
+    for (int i = 3; i >= 0; i--) if (k[i] != FR_R[i]) return k[i] < FR_R[i];
+    return false;
+}
+bool fr_zero(const uint64_t *k) { return !(k[0] | k[1] | k[2] | k[3]); }
+// the trapdoor and everything derived from it (powers of tau, Lagrange coefficients, at / bt / ct, the query scalars) is the
+// setup's toxic waste: the staging buffers that held it are cleared however the call ends
+struct ClearTrapdoor {
+    zk_ctx *ctx;
+    ~ClearTrapdoor() {
+        for (DevBuf *b : {&ctx->g_a, &ctx->g_b, &ctx->g_c, &ctx->g_h, &ctx->g_scal, &ctx->g_scal2, &ctx->ntt_tmp})
+            if (b->p) cudaMemsetAsync(b->p, 0, b->cap, ctx->stream);
+        cudaStreamSynchronize(ctx->stream);
+    }
+};
+}  // namespace
+
+extern "C" int zk_groth16_generate(zk_ctx *ctx, const zk_r1cs *q, const uint8_t g1[96], const uint8_t g2[192], const uint64_t alpha[4],
+                                   const uint64_t beta[4], const uint64_t gamma[4], const uint64_t delta[4], const uint64_t tau[4], zk_params **out) {
+    if (!ctx || !q || !g1 || !g2 || !alpha || !beta || !gamma || !delta || !tau || !out) { zk_set_error("zk_groth16_generate: NULL argument"); return ZK_ERR_INVALID; }
+    if (q->device != ctx->device) { zk_set_error("constraint system lives on device %d, context on %d", q->device, ctx->device); return ZK_ERR_INVALID; }
+    const uint64_t *sc[5] = {tau, alpha, beta, gamma, delta};
+    static const char *names[5] = {"tau", "alpha", "beta", "gamma", "delta"};
+    for (int k = 0; k < 5; k++) if (!fr_canonical(sc[k])) { zk_set_error("%s is not canonical (>= r)", names[k]); return ZK_ERR_NOT_CANONICAL; }
+    // gamma, delta: bellman's own UnexpectedIdentity; alpha, beta: zk_params_load would reject the vk points; tau: the h query would
+    // hold the identity, which Parameters::read rejects
+    for (int k : {3, 4, 1, 2, 0}) if (fr_zero(sc[k])) { zk_set_error("UnexpectedIdentity: %s = 0", names[k]); return ZK_ERR_UNEXPECTED_IDENTITY; }
+    ZK_TRY(zk_use_device(ctx));
+    const size_t n_c = q->n_c, n_in = q->n_in, n_aux = q->n_aux, nv = n_in + n_aux;
+    unsigned log_m = 0;
+    size_t m = 1;
+    while (m < n_c + n_in) { m <<= 1; log_m++; }
+    if (log_m > 28 || m - 1 >= CRS_POINT_LIMIT || nv >= CRS_POINT_LIMIT) {
+        zk_set_error("PolynomialDegreeTooLarge: domain 2^%u, %zu variables (limits 2^28, %u points per vector)", log_m, nv, CRS_POINT_LIMIT);
+        return ZK_ERR_POLY_DEGREE_TOO_LARGE;
+    }
+    ClearTrapdoor clear{ctx};
+    cudaStream_t st = ctx->stream;
+    // ---- staging (reserved up front: a buffer that grows later would be freed without being cleared) ----
+    const size_t nnz_max = q->nnz[0] > q->nnz[1] ? (q->nnz[0] > q->nnz[2] ? q->nnz[0] : q->nnz[2]) : (q->nnz[1] > q->nnz[2] ? q->nnz[1] : q->nnz[2]);
+    const size_t g1_cap = m + n_aux + 2 * (nv + 2) + 3 + n_in + 8;
+    ZK_TRY(ctx->g_a.reserve(m * 32));                        // powers of tau, then the Lagrange coefficients
+    ZK_TRY(ctx->ntt_tmp.reserve(m * 32));
+    ZK_TRY(ctx->g_h.reserve((3 * nv + 16) * 32));            // at | bt | ct, the constants, the five scalars
+    ZK_TRY(ctx->g_b.reserve((nnz_max + nv + 1) * 32));       // column-sorted entries and task sums (ping-pong)
+    ZK_TRY(ctx->g_c.reserve((nnz_max + nv + 1) * 32));
+    ZK_TRY(ctx->g_scal.reserve(g1_cap * 32));                // G1 scalars in CrsLayout order
+    ZK_TRY(ctx->g_scal2.reserve((nv + 8) * 32));             // G2 scalars
+    auto rnd = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t scratch_words = 3 * (nv + 1) + 2 * (nv / 2048 + 8) + 64;
+    ZK_TRY(ctx->g_misc.reserve(rnd(288) + rnd(sizeof(G1Affine)) + rnd(sizeof(G2Affine)) + rnd(16) + 3 * rnd((nv + 1) * 4) + rnd(scratch_words * 4)));
+    uint8_t *mp = ctx->g_misc.as<uint8_t>();
+    auto carve = [&](size_t bytes) { uint8_t *r = mp; mp += rnd(bytes); return r; };
+    uint8_t *d_enc = carve(288);
+    G1Affine *d_gen1 = (G1Affine *)carve(sizeof(G1Affine));
+    G2Affine *d_gen2 = (G2Affine *)carve(sizeof(G2Affine));
+    int *d_flag = (int *)carve(16);
+    uint32_t *pos_a = (uint32_t *)carve((nv + 1) * 4), *pos_b = (uint32_t *)carve((nv + 1) * 4), *scratch = (uint32_t *)carve(scratch_words * 4);
+    uint4 *abc = ctx->g_h.as<uint4>(), *consts = abc + 2 * 3 * nv, *d_in = consts + 2 * 8;
+    uint4 *P = ctx->g_a.as<uint4>(), *scal1 = ctx->g_scal.as<uint4>(), *scal2 = ctx->g_scal2.as<uint4>();
+    // ---- generators: checked decoding (on the curve, in the r-torsion, not the identity) ----
+    ZK_CUDA(cudaMemcpyAsync(d_enc, g1, 96, cudaMemcpyHostToDevice, st));
+    ZK_CUDA(cudaMemcpyAsync(d_enc + 96, g2, 192, cudaMemcpyHostToDevice, st));
+    zkcodec::k_decode_uncompressed<Fq><<<1, 128, 0, st>>>(d_enc, 1, 1, 1, d_gen1, ctx->d_err + 1);
+    zkcodec::k_decode_uncompressed<Fq2><<<1, 128, 0, st>>>(d_enc + 96, 1, 1, 1, d_gen2, ctx->d_err + 1);
+    ZK_CUDA(cudaGetLastError());
+    ZK_TRY(zk_check_err_flag(ctx));
+    // ---- powers of tau, h, Lagrange coefficients ----
+    for (int k = 0; k < 5; k++) ZK_CUDA(cudaMemcpyAsync(d_in + 2 * k, sc[k], 32, cudaMemcpyHostToDevice, st));
+    ZK_CUDA(cudaMemsetAsync(d_flag, 0, 16, st));
+    ZK_TRY(zk_setup_powers(ctx, d_in, log_m, consts, d_flag, P, scal1));        // h = G1 scalars [0, m - 1) (CrsLayout: o_h = 0)
+    int flags[2] = {0, 0};
+    ZK_CUDA(cudaMemcpyAsync(flags, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    ZK_CUDA(cudaStreamSynchronize(st));
+    if (flags[0]) { zk_set_error("UnexpectedIdentity: tau^m = 1 (m = 2^%u), the h query would contain the identity", log_m); return ZK_ERR_UNEXPECTED_IDENTITY; }
+    ZK_TRY(zk_ntt_run(ctx, P, log_m, ZK_NTT_IFFT, 1));
+    // ---- at, bt, ct (the `input_i * 0 = 0` rows add L_{n_c + i} to at) ----
+    for (int w = 0; w < 3; w++)
+        ZK_TRY(zk_setup_qap(ctx, q->d_row_ptr[w], q->d_col[w], q->d_coeff[w], n_c, q->nnz[w], nv, P, w == 0 ? n_in : 0, scratch,
+                            ctx->g_b.p, ctx->g_c.p, abc + 2 * w * nv));
+    // ---- query sizes: identities dropped from a, b_g1, b_g2 by value; an l scalar of zero is an unconstrained variable ----
+    ZK_TRY(zk_setup_flags(ctx, abc, consts, nv, n_in, pos_a, pos_b, d_flag + 1, scratch));
+    uint32_t cnt_ab[2] = {0, 0};
+    ZK_CUDA(cudaMemcpyAsync(cnt_ab, pos_a + nv, 4, cudaMemcpyDeviceToHost, st));
+    ZK_CUDA(cudaMemcpyAsync(cnt_ab + 1, pos_b + nv, 4, cudaMemcpyDeviceToHost, st));
+    ZK_CUDA(cudaMemcpyAsync(flags + 1, d_flag + 1, 4, cudaMemcpyDeviceToHost, st));
+    ZK_CUDA(cudaStreamSynchronize(st));
+    if (flags[1]) { zk_set_error("UnconstrainedVariable: an aux variable's l query point is the identity"); return ZK_ERR_UNCONSTRAINED_VARIABLE; }
+    const size_t cnt[6] = {n_in, m - 1, n_aux, cnt_ab[0], cnt_ab[1], cnt_ab[1]};
+    CrsLayout L(cnt);
+    // ---- the scalars in CrsLayout order: h' | l | a' | b_g1' | vk1 and b_g2' | vk2 ----
+    auto put = [&](uint4 *dst, int k) { return cudaMemcpyAsync(dst, d_in + 2 * k, 32, cudaMemcpyDeviceToDevice, st); };
+    enum { TAU, ALPHA, BETA, GAMMA, DELTA };
+    ZK_CUDA(put(scal1 + 2 * (L.o_h + m - 1), DELTA));
+    ZK_CUDA(put(scal1 + 2 * (L.o_a + cnt[3]), ALPHA)); ZK_CUDA(put(scal1 + 2 * (L.o_a + cnt[3] + 1), DELTA));
+    ZK_CUDA(put(scal1 + 2 * (L.o_b1 + cnt[4]), BETA)); ZK_CUDA(put(scal1 + 2 * (L.o_b1 + cnt[4] + 1), DELTA));
+    ZK_CUDA(put(scal1 + 2 * L.o_vk1, ALPHA)); ZK_CUDA(put(scal1 + 2 * (L.o_vk1 + 1), BETA)); ZK_CUDA(put(scal1 + 2 * (L.o_vk1 + 2), DELTA));
+    ZK_CUDA(put(scal2 + 2 * cnt[5], BETA)); ZK_CUDA(put(scal2 + 2 * (cnt[5] + 1), DELTA));
+    ZK_CUDA(put(scal2 + 2 * (L.n_b2), BETA)); ZK_CUDA(put(scal2 + 2 * (L.n_b2 + 1), GAMMA)); ZK_CUDA(put(scal2 + 2 * (L.n_b2 + 2), DELTA));
+    ZK_TRY(zk_setup_fill(ctx, abc, consts, nv, n_in, pos_a, pos_b, scal1 + 2 * L.o_l, scal1 + 2 * (L.o_vk1 + 3), scal1 + 2 * L.o_a, scal1 + 2 * L.o_b1, scal2));
+    // ---- the group elements: one fixed-base launch per group ----
+    ZK_TRY(ctx->stage_b.reserve((L.g1_total + 8) * sizeof(G1Affine)));
+    ZK_TRY(ctx->stage_c.reserve((L.g2_total + 8) * sizeof(G2Affine)));
+    ZK_TRY(zk_fixed_base(ctx, 1, d_gen1, scal1, L.g1_total, ctx->stage_b.p));
+    ZK_TRY(zk_fixed_base(ctx, 2, d_gen2, scal2, L.g2_total, ctx->stage_c.p));
+    ZK_TRY(params_from_device(ctx, L, ctx->stage_b.as<G1Affine>(), ctx->stage_c.as<G2Affine>(), out));
+    (*out)->subgroup_checked = true;     // every point is a multiple of a checked generator
     return ZK_OK;
 }

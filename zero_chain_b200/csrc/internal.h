@@ -78,6 +78,7 @@ struct zk_ctx {
     DevBuf g_scal3;                // A-query scalars
     zk_ctx *aux = nullptr;         // second lane (own stream + workspace) on the same device: the prover's G2 MSM overlaps the G1 work
     DevBuf g_scal2;                // B-query scalars (shared by the G1 and G2 B MSMs)
+    DevBuf fb_tbl;                 // table of the batched fixed-base multiplication (setup.cu)
     // asynchronous MSM (zk_msm_begin / zk_msm_end): everything after the bucket accumulation runs on a HIGH-PRIORITY stream, so that
     // with two contexts in flight the latency-bound tail of one MSM is scheduled ahead of the other's accumulation blocks
     cudaStream_t tail = nullptr;
@@ -120,5 +121,14 @@ void zk_launch_miller_lanes(cudaStream_t st, size_t n, const void *a, const void
 void zk_launch_verify_final_lanes(cudaStream_t st, size_t n, const void *f, const void *alpha_beta, const uint8_t *status, uint8_t *verdict);
 int zk_fr_to_mont(zk_ctx *ctx, const void *d_in, size_t n, void *d_out);
 int zk_fr_witness_to_mont(zk_ctx *ctx, const void *d_inputs, size_t n_in, const void *d_aux, size_t n_aux, size_t batch, void *d_z);
+// parameter generation and the batched fixed-base multiplication (setup.cu)
+int zk_fixed_base(zk_ctx *ctx, int group, const void *d_base, const void *d_scalars, size_t n, void *d_out);
+int zk_setup_powers(zk_ctx *ctx, const void *d_in, unsigned log_m, void *d_consts, int *d_flag, void *d_P, void *d_h);
+int zk_setup_qap(zk_ctx *ctx, const uint32_t *d_row_ptr, const uint32_t *d_col, const void *d_coeff, size_t n_c, size_t nnz, size_t nv,
+                 const void *d_L, size_t n_in_rows, uint32_t *scratch, void *d_vals0, void *d_vals1, void *d_out);
+int zk_setup_flags(zk_ctx *ctx, const void *d_abc, const void *d_consts, size_t nv, size_t n_in, uint32_t *pos_a, uint32_t *pos_b, int *d_flag,
+                   uint32_t *scratch);
+int zk_setup_fill(zk_ctx *ctx, const void *d_abc, const void *d_consts, size_t nv, size_t n_in, const uint32_t *pos_a, const uint32_t *pos_b,
+                  void *d_l, void *d_ic, void *d_a, void *d_b1, void *d_b2);
 int zk_fr_r1cs_eval(zk_ctx *ctx, const uint32_t *d_row_ptr, const uint32_t *d_col, const void *d_coeff, const void *d_z, size_t n_c, size_t n_in,
                     size_t nv, unsigned log_m, int which, size_t batch, void *d_dst);

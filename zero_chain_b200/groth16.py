@@ -6,6 +6,7 @@ Names follow upstream bellman 0.1.0 as the reference uses them:
   multiexp(bases, exponents)         bellman::multiexp::multiexp  (SURVEY.md §3.2)
   EvaluationDomain.{fft,ifft,coset_fft,icoset_fft}   bellman::domain (SURVEY.md §8 a7)
   Proof (192-byte wire form)         core/bellman-verifier/src/lib.rs:40-110
+  generate_random_parameters         core/proofs/src/setup.rs:28,59
 Errors mirror bellman::SynthesisError (zface/src/error.rs:17,45-48).
 
 All numeric arrays are numpy uint64 little-endian limbs: Fr canonical (n,4) at this boundary,
@@ -28,7 +29,7 @@ R_MODULUS = 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001
 class SynthesisError(Exception):
     """bellman::SynthesisError variants reachable from the prover path."""
     NAMES = {-3: "AssignmentMissing", -4: "PolynomialDegreeTooLarge", -5: "UnexpectedIdentity", -6: "IoError",
-             -7: "IoError(GroupDecodingError)", -8: "IoError(NotInField)", -9: "MalformedVerifyingKey"}
+             -7: "IoError(GroupDecodingError)", -8: "IoError(NotInField)", -9: "MalformedVerifyingKey", -10: "UnconstrainedVariable"}
 
     def __init__(self, code, msg):
         super().__init__("%s: %s" % (self.NAMES.get(code, "Error(%d)" % code), msg))
@@ -491,6 +492,46 @@ def create_proof_from_witness_batch(cs: ConstraintSystem, params: Parameters, ba
     out = np.zeros(192 * batch, np.uint8)
     _ck(_lib.lib().zk_groth16_prove_witness_batch(params.ctx._h, params._h, cs._h, batch, _p(inputs), _p(aux), _p(r), _p(s), _p(out)))
     return out.tobytes()
+
+
+def generate_parameters(cs: ConstraintSystem, g1: bytes, g2: bytes, alpha: int, beta: int, gamma: int, delta: int, tau: int) -> Parameters:
+    """groth16::generate_parameters(circuit, g1, g2, alpha, beta, gamma, delta, tau) for the constraint system `cs` on its device.
+    g1 / g2: G1Uncompressed (96 B) / G2Uncompressed (192 B) generators; the five scalars canonical.  The result is resident and ready
+    to prove with; its write() is the byte stream bellman's Parameters::write emits for the same inputs."""
+    g1, g2 = np.frombuffer(bytes(g1), np.uint8), np.frombuffer(bytes(g2), np.uint8)
+    assert g1.size == 96 and g2.size == 192
+    sc = [_fr_limbs(x) if 0 <= x < 1 << 256 else None for x in (alpha, beta, gamma, delta, tau)]
+    if any(x is None for x in sc):
+        raise SynthesisError(-8, "scalar outside [0, 2^256)")
+    h = C.c_void_p()
+    _ck(_lib.lib().zk_groth16_generate(cs.ctx._h, cs._h, _p(g1), _p(g2), *[_p(x) for x in sc], C.byref(h)))
+    cnt = np.zeros(6, np.uint64)
+    _ck(_lib.lib().zk_params_counts(h, _p(cnt)))
+    return Parameters(cs.ctx, h, [int(x) for x in cnt])
+
+
+def generate_random_parameters(cs: ConstraintSystem, rng=None) -> Parameters:
+    """groth16::generate_random_parameters: g1, g2 uniform non-identity group elements (random non-zero multiples of the
+    standard generators, which is what G1::rand / G2::rand give in a group of prime order), then alpha, beta, gamma, delta, tau
+    uniform in Fr (Fr::rand), drawn in bellman's order; `rng` as for create_random_proof."""
+    from .synthetic import g1_limbs_to_uncompressed, g2_limbs_to_uncompressed
+    draw = (lambda: secrets.randbelow(R_MODULUS)) if rng is None else (lambda: rng.randrange(R_MODULUS))
+    k1, k2 = 1 + draw() % (R_MODULUS - 1), 1 + draw() % (R_MODULUS - 1)
+    g1 = g1_limbs_to_uncompressed(scalar_mul_many(cs.ctx, 1, G1_GENERATOR, [_fr_limbs(k1)])[0])
+    g2 = g2_limbs_to_uncompressed(scalar_mul_many(cs.ctx, 2, G2_GENERATOR, [_fr_limbs(k2)])[0])
+    alpha, beta, gamma, delta, tau = (draw() for _ in range(5))
+    return generate_parameters(cs, g1, g2, alpha, beta, gamma, delta, tau)
+
+
+def parameter_files(params: Parameters):
+    """The two files of the reference's write_to_file (core/proofs/src/crypto_components.rs:277): the proving key
+    (Parameters::write, e.g. conf_pk.dat) and the prepared verifying key (PreparedVerifyingKey::write of
+    prepare_verifying_key(&params.vk), e.g. conf_vk.dat)."""
+    pvk = PreparedVerifyingKey.prepare(params.ctx, params.vk_bytes())
+    try:
+        return params.write(), pvk.write()
+    finally:
+        pvk.free()
 
 
 def create_proof_batch_raw(params: Parameters, batch: int, a, b, c, inputs, aux, a_aux_density, b_input_density, b_aux_density, r, s) -> bytes:
